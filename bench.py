@@ -17,6 +17,10 @@ Workloads (BASELINE.json `configs`; the default is the headline, configs[2]):
 A "step" is one pass of the hot path over one batch (streams: --stream-frames consecutive frames of every stream).
 `value` is whole-job frames/s with the batch resident in HBM; `e2e` is the same work through the C ABI on pinned
 HOST frames (H2D + D2H inside the timed region).
+
+--dump-outputs DIR writes what the last timed step returned as DIR/<name>.npy (float64, frame or stream index first;
+rank 0's share with --gpus > 1), plus frame_index.npy naming the frames the files hold.  The inputs depend only on the
+arguments, so two builds of the library can be compared output for output.
 """
 import argparse
 import json
@@ -31,6 +35,7 @@ from pathlib import Path
 import numpy as np
 
 ROOT = Path(__file__).resolve().parent
+sys.dont_write_bytecode = True      # the tree may be read-only: the benchmark leaves no bytecode caches in it
 sys.path.insert(0, str(ROOT))
 
 from headtrackr_b200 import synth  # noqa: E402
@@ -87,6 +92,45 @@ def captured_traffic(W, H):
     except Exception:
         pass
     return None, None
+
+
+DUMP_LIMIT = 64 << 20       # bytes --dump-outputs may write in all
+
+
+def step_outputs(workload, rects, counts, found, objs, wins, events):
+    """The records one step of `workload` returns, decoded from the C structs (include/headtrackr_b200.h) into float64
+    arrays with the frame (streams: stream) index first.  Rect rows past a frame's count hold no result and are zeroed."""
+    if workload == "streams":
+        ev = events.cpu().numpy()                       # (T, B, 56) ht_stream_event
+        dec = np.concatenate([ev.view(np.int32)[..., :2].astype(np.float64), ev.view(np.float64)[..., 1:7]], axis=-1)
+        return {"events": dec.transpose(1, 0, 2)}       # detection, status, x, y, width, height, angle, confidence
+    n = counts.cpu().numpy()
+    r = rects.cpu().numpy()                             # (B, K, 6) ht_rect
+    r = np.concatenate([r[..., :5], r.view(np.int32)[..., 10:11].astype(np.float64)], axis=-1)  # ..., confidence, neighbors
+    r[np.arange(r.shape[1])[None, :] >= n[:, None]] = 0.0
+    out = {"rects": r, "counts": n.astype(np.float64)}
+    if workload == "detect_track30":
+        o = objs.cpu().numpy()                          # (B, 6) int32 = ht_trackobj: x, y, width, height, fp64 angle
+        out.update(found=found.cpu().numpy().astype(np.float64),
+                   objs=np.concatenate([o[:, :4].astype(np.float64), np.ascontiguousarray(o[:, 4:6]).view(np.float64)], axis=1),
+                   windows=wins.cpu().numpy().astype(np.float64))
+    return out
+
+
+def write_outputs(out_dir, arrays, limit=DUMP_LIMIT):
+    """DIR/<name>.npy for every array and DIR/frame_index.npy, the frames they hold: all of them, or a fixed, seeded
+    sample when all of them would exceed `limit` bytes."""
+    n = len(next(iter(arrays.values())))
+    per_frame = sum(a[0].nbytes for a in arrays.values()) + 8
+    room = limit - 128 * (len(arrays) + 1)              # .npy headers
+    keep = np.arange(n)
+    if n * per_frame > room:
+        keep = np.sort(np.random.default_rng(0).choice(n, room // per_frame, replace=False))
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    np.save(out_dir / "frame_index.npy", keep.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(out_dir / f"{name}.npy", np.ascontiguousarray(a[keep]))
 
 
 class ClockSampler:
@@ -462,6 +506,8 @@ def run_ours(args, cfg):
     e1.record(stream)
     barrier()
     ms_local = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:     # before the measurements below reuse the output buffers
+        write_outputs(args.dump_outputs, step_outputs(workload, *last_outputs(), d_events))
     prof = ctx.profile_read(reset=True)
     ctx.profile(False)
     track_stats = ctx.debug_track_stats(reset=True)
@@ -733,7 +779,13 @@ def main():
     ap.add_argument("--pipeline", type=int, default=int(os.environ.get("HT_BENCH_PIPELINE", "0")),
                     help="detect+track: 0 (default) = every step joins its own tracking, 1 = pipelined steps "
                          "(ht_set_pipeline); on one GPU the other mode is measured too and reported beside the headline")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the CUDA path (--impl ours)")
     cfg = dict(WORKLOADS[args.workload], workload=args.workload, stream_frames=args.stream_frames)
     for k, v in (("width", args.width), ("height", args.height), ("interval", args.interval),
                  ("batch", args.streams if args.streams is not None else args.batch)):

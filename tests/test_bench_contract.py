@@ -45,6 +45,27 @@ def test_gpu_arm_has_no_cpu_fallback():
     assert "no CUDA device" in (p.stderr + p.stdout)
 
 
+def test_bad_step_counts_are_refused():
+    for args in (("--steps", "0"), ("--warmup", "-1")):
+        p = run_bench("--impl", "reference", *args)
+        assert p.returncode == 2 and "--steps must be at least 1" in p.stderr
+
+
+def test_dump_outputs_above_the_limit_is_a_fixed_sample(tmp_path):
+    sys.path.insert(0, str(ROOT))
+    import bench
+    import numpy as np
+    arrays = {"rects": np.arange(1000 * 16, dtype=np.float64).reshape(1000, 16), "counts": np.arange(1000.0)}
+    for d in ("a", "b"):
+        bench.write_outputs(tmp_path / d, arrays, limit=40_000)
+    idx = np.load(tmp_path / "a" / "frame_index.npy")
+    assert 0 < len(idx) < 1000 and np.all(np.diff(idx) > 0)
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= 40_000
+    for name, a in arrays.items():
+        got = np.load(tmp_path / "a" / f"{name}.npy")
+        assert np.array_equal(got, a[idx.astype(int)]) and np.array_equal(got, np.load(tmp_path / "b" / f"{name}.npy"))
+
+
 def test_usable_cores_is_bounded_by_the_affinity_mask():
     sys.path.insert(0, str(ROOT))
     import bench

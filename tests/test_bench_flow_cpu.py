@@ -204,9 +204,32 @@ def test_single_rank_line(pipeline):
                 "vs_baseline", "dtype", "data", "config", "e2e", "gpu_launches", "roofline", "clocks"):
         assert key in line, key
     assert line["n_gpus"] == 1 and line["steps"] == 3 and line["value"] > 0
+    assert line["gpu_launches"] == 3                                # the fake launches once per step: 3 timed steps
     other = "unpipelined" if pipeline else "pipelined"
     assert other in line and "error" not in line[other] and line[other]["value"] > 0
     assert line["config"]["pipeline"].startswith("on" if pipeline else "off")
+
+
+@pytest.mark.parametrize("pipeline", [0, 1])
+def test_dump_outputs_hold_the_last_timed_step(pipeline, tmp_path):
+    """--dump-outputs: the records of the last timed step (pipelined: once its tracking has been joined, not the -1
+    placeholders of a step still in flight), as float64, identical on a second run."""
+    sys.path.insert(0, str(ROOT))
+    import bench
+    base = bench.make_base_frames(64, 48, 0, bench.N_UNIQUE)
+    want = [checksum(np.roll(base[j % bench.N_UNIQUE], (j // bench.N_UNIQUE) * 16, axis=1)) for j in range(8)]
+    dirs = [tmp_path / "a", tmp_path / "b"]
+    for d in dirs:
+        launch(1, SMALL + ["--pipeline", str(pipeline), "--dump-outputs", str(d)])
+    names = sorted(p.name for p in dirs[0].iterdir())
+    assert names == ["counts.npy", "found.npy", "frame_index.npy", "objs.npy", "rects.npy", "windows.npy"]
+    got = {n: np.load(dirs[0] / n) for n in names}
+    assert all(a.dtype == np.float64 and len(a) == 8 for a in got.values())
+    assert got["frame_index.npy"].tolist() == list(range(8))
+    assert got["objs.npy"].shape == (8, 5) and got["objs.npy"][:, 0].tolist() == want
+    assert got["rects.npy"].shape == (8, FakeContext.K, 6)
+    for n in names:
+        assert np.array_equal(got[n], np.load(dirs[1] / n)), n
 
 
 @pytest.mark.parametrize("pipeline,workload", [(0, "detect_track30"), (1, "detect_track30"), (0, "detect")])
@@ -221,10 +244,14 @@ def test_two_ranks_same_collectives_and_right_records(pipeline, workload):
     assert len(line["per_rank"]) == 2 and line["gather"]["overlapped"] is True
 
 
-def test_two_ranks_streams_workload():
-    """config 5's loop (one ht_stream_step per video frame, T frames per step) on two skewed ranks."""
+def test_two_ranks_streams_workload(tmp_path):
+    """config 5's loop (one ht_stream_step per video frame, T frames per step) on two skewed ranks; --dump-outputs
+    holds rank 0's event records of the last step, stream-major."""
     argv = ["--width", "64", "--height", "48", "--streams", "2", "--stream-frames", "4", "--steps", "2", "--warmup", "3",
-            "--no-cpu-baseline", "--gpus", "2", "--workload", "streams"]
+            "--no-cpu-baseline", "--gpus", "2", "--workload", "streams", "--dump-outputs", str(tmp_path)]
     outs = launch(2, argv, skew=0.15)
     line = json.loads(outs[0].strip().splitlines()[-1])
     assert line["n_gpus"] == 2 and line["value"] > 0 and "streams" in line
+    assert sorted(p.name for p in tmp_path.iterdir()) == ["events.npy", "frame_index.npy"]
+    ev = np.load(tmp_path / "events.npy")
+    assert ev.dtype == np.float64 and ev.shape == (2, 4, 8)
