@@ -290,7 +290,7 @@ int parse_cascade(const void *blob, size_t len, HostCascade &hc, std::string &er
   auto point_off = [&](int z, int x, int y, bool &ok) -> uint16_t {
     const int lim = (24 >> z) - 1;
     if (z < 0 || z > 2 || x < 0 || y < 0 || x > lim || y > lim) { ok = false; return 0; }
-    return (uint16_t)(point_word(z, x, y) | ((z > 0 && !HT_UNIBASE) ? 0x8000 : 0));   // bit 15: relative to baseB (two-base layout)
+    return (uint16_t)(point_word(z, x, y) | (z > 0 ? 0x8000 : 0));   // bit 15: relative to baseB
   };
   for (int k = 0; k < hc.n_features; ++k) {
     const uint8_t *r = pf + (size_t)k * 32;
@@ -340,13 +340,7 @@ int parse_cascade(const void *blob, size_t len, HostCascade &hc, std::string &er
   // numbers are not 8-digit decimals, lane-per-window groups to the end.
   {
     int g = 0;
-#if HT_GROUP_SPLIT >= 2
-    const int cuts_fast[] = {0, 2, 3, 4, 5, 6, 7};   // {0,1} {2} {3} {4} {5} {6} {7}
-#elif HT_GROUP_SPLIT == 1
-    const int cuts_fast[] = {0, 2, 3, 4, 5, 6};      // {0,1} {2} {3} {4} {5} {6,7}
-#else
     const int cuts_fast[] = {0, 2, 3, 4, 6};         // {0,1} {2} {3} {4,5} {6,7}: the generated stages
-#endif
     const int cuts_int[] = {0, 2, 4, 6};
     const int cuts_fp[] = {0, 2, 4, 6, 9};
     static_assert(HT_GEN_STAGES == 8, "cuts_fast assumes 8 generated stages");
@@ -508,12 +502,9 @@ struct ht_ctx {
   // buffered by call parity (bin planes, current-frame histograms) or ordered by an event (the caller's rectangle
   // arrays: k_group of call s+1 waits for the tracking of call s).  Every other entry point joins first.
   int pipeline = 0;
-  int pipe_bg = 0;                          // HT_PIPE_BG=1: pipelined tracking runs BELOW the priority of the context's stream,
-                                            // and k_cascade leaves room for one k_track CTA per SM while it is in flight
   bool aux_pending = false;                 // work on aux_stream that the context's stream has not waited for yet
   cudaEvent_t pipe_detect_done = nullptr;
   int pipe_parity = 0;
-  cudaStream_t main_stream = nullptr;       // the context's stream while ctx->stream is temporarily the aux stream
   size_t bins_off = 0, hist_off = 0;        // element offsets of the active bin-plane / histogram buffer (parity)
   // Tracking of part p on a second stream while part p+1 is uploaded / detected (ht_detect_track).  Default (-1):
   // only for HOST frames, where the batch arrives at PCIe speed and the GPU has idle time to fill - measured e2e
@@ -541,34 +532,27 @@ struct ht_ctx {
   cudaEvent_t compute_done = nullptr;
   std::vector<cudaEvent_t> chunk_events;
   int h2d_chunk = 64;                       // frames per pipelined upload chunk
-  int track_cluster = 0;                    // >0: force single-phase k_track with that cluster size (A/B profiling)
+  int track_cluster = 0;                    // >0: force that k_track cluster size, 2, 4 or 8 (HT_TRACK_CLUSTER, A/B profiling)
   bool track_memo = true;                   // k_track re-uses the moments of windows it has already summed in this
                                             // launch (ht_set_track_memo / HT_TRACK_MEMO=0 for the strict A/B)
   bool track_trace = false;                 // HT_TRACK_TRACE=1: k_track writes a per-stream timeline (ht_debug_track_trace)
   DevBuf d_trace;
-  int track_nt = 256;                       // threads per k_track CTA (HT_TRACK_NT=128|256)
   bool track_lpt = true;                    // longest-chain-first launch order (HT_TRACK_LPT=0 disables)
   DevBuf d_stream_mode, d_stream_mask, d_stream_cs, d_stream_init, d_stream_events;   // ht_stream_step
   DevBuf d_head_state, d_head_params, d_head_events;                                  // ht_stream_head_config
   bool head_on = false;
-  bool track_history = true;                // order by the cost of each stream's previous launch (HT_TRACK_HISTORY=0: by window area)
   DevBuf d_track_cost;                      // [max_frames][2] {passes, window pixels / 256} per slot
-  int track_heavy_div = 128;                // >0: the n/div costliest streams run on a cluster of
-  int track_heavy_cluster = 8;              //     track_heavy_cluster CTAs on sched_stream (HT_TRACK_HEAVY=div[,cluster])
+  int track_heavy_div = 128;                // >0: the n/div costliest streams run on clusters of
+  int track_heavy_cluster = 8;              //     track_heavy_cluster CTAs (HT_TRACK_HEAVY=div[,cluster])
   int track_mid_div = 32, track_mid_cluster = 4;  // HT_TRACK_MID=div[,cluster]: the next n/32 costliest streams on clusters of 4
                                                   // (call 4: 4.12 -> 3.40 ms per 1024 x 30 calls with n/16; call 17, with
                                                   // prioritised tier streams: n/64 + n/16 3.17, n/128 + n/32 2.97, n/64 + n/48 3.00)
-  double track_light_div = 0; int track_light_nt = 256;  // HT_TRACK_LIGHT=div[,threads]: the cheapest n/div streams (div may be fractional) on single CTAs
-  cudaStream_t tier_stream[4] = {nullptr, nullptr, nullptr, nullptr};   // heavy, mid, light, rest (side 3: when tiers are on)
-  cudaEvent_t tier_done[4] = {nullptr, nullptr, nullptr, nullptr};
+  cudaStream_t tier_stream[3] = {nullptr, nullptr, nullptr};   // heavy, mid, rest
+  cudaEvent_t tier_done[3] = {nullptr, nullptr, nullptr};
   int track_mask_frames = 4;                // >0: mask only streams whose last launch swept more than this many frames' worth of pixels
   int track_mask_min = 4;                   // HT_TRACK_MASK=<min n_calls> (0: off): zero-weight marking of the bin plane before k_track
-  int track_prio = 1;                       // HT_TRACK_PRIO=0: tier streams without priorities, the default tier on the context's stream
-  cudaStream_t sched_stream = nullptr;
-  cudaEvent_t sched_ready = nullptr, sched_done = nullptr;
-  int track_bail_area = 0;                  // >0: two-phase k_track; phase A hands streams with a larger window (px) to phase B
-  DevBuf d_sched;                           // k_track two-phase scheduling scratch
-  unsigned sched_seq = 0;
+  cudaEvent_t sched_ready = nullptr;
+  DevBuf d_sched;                           // k_track launch-order scratch: [area | order][max_frames]
 
   int fail(int code, const char *fmt, ...) {
     char buf[512];
@@ -669,7 +653,7 @@ int ensure_tracker_buffers(ht_ctx *ctx) {
     CK(ctx->d_found.reserve(mf * sizeof(int32_t)));
     CK(ctx->d_objs.reserve(mf * 6 * sizeof(int32_t)));
     CK(ctx->d_windows.reserve(mf * 4 * sizeof(int32_t)));
-    CK(ctx->d_sched.reserve((2 * mf + 64) * sizeof(int32_t)));
+    CK(ctx->d_sched.reserve(2 * mf * sizeof(int32_t)));
     CK(ctx->d_track_cost.reserve(2 * mf * sizeof(int32_t)));
     CK(cudaMemsetAsync(ctx->d_track_cost.p, 0, 2 * mf * sizeof(int32_t), ctx->stream));
     if (ctx->track_trace) {   // [mf x 4] per-stream records, then [mf x 8] phase totals (HT_TRACK_PASSTRACE builds)
@@ -694,10 +678,6 @@ int launch_hist(ht_ctx *ctx, const uint8_t *d_rgba, int n, int w, int h, uint32_
   return HT_OK;
 }
 
-// k_track runs in two phases.  Phase A: one CTA per stream (no cluster overhead) — streams whose search window
-// outgrows bail_area stop and are queued.  Phase B: one 8-CTA cluster per queued stream finishes their calls.
-// Mean-shift is a serial chain of window passes per stream, so the few streams with large windows would
-// otherwise set the duration of the whole launch.
 // per-launch options of k_track that do not depend on the batch
 struct TrackOpts {
   unsigned long long *trace;   // HT_TRACK_TRACE=1: per-stream timeline buffer (else NULL)
@@ -708,64 +688,43 @@ struct TrackOpts {
   const uint8_t *enable;       // ht_stream_step: per stream, 0 = not tracking this frame (else NULL)
 };
 
-template <int C, int NT = 256>
+template <int C>
 cudaError_t launch_track_c(cudaStream_t st, int n, const uint16_t *bins, int w, int h, const int32_t *d_slots,
                            const uint32_t *mh, const uint32_t *ch, TrackState *state, int n_calls, int32_t *d_objs,
-                           int32_t *d_win, int32_t *flag, unsigned long long *stats, int bail_area, int32_t *calls_done,
-                           int32_t *bail_list, int32_t *bail_count, int use_list, int list_off, TrackOpts opt) {
+                           int32_t *d_win, int32_t *flag, unsigned long long *stats, const int32_t *order, int list_off,
+                           TrackOpts opt) {
   // Same shared-memory carve-out as k_cascade (the maximum): an SM only changes its L1 / shared split when it is idle,
   // so CTAs of kernels that ask for different splits do not mix on one SM - and k_track is meant to run beside the
   // detection kernels of the next call (ht_set_pipeline).
   static bool carveout_set = false;
   if (!carveout_set) {
-    cudaError_t ce = cudaFuncSetAttribute(k_track<C, NT>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+    cudaError_t ce = cudaFuncSetAttribute(k_track<C>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
     if (ce != cudaSuccess) return ce;
     carveout_set = true;
   }
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3((unsigned)n * C);
-  cfg.blockDim = dim3(NT);
+  cfg.blockDim = dim3(TRACK_THREADS);
   cfg.dynamicSmemBytes = 0;
   cfg.stream = st;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
   attr[0].val.clusterDim.x = C; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr; cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, k_track<C, NT>, bins, w, h, d_slots, mh, ch, state, n_calls, d_objs, d_win, flag, stats,
-                            bail_area, calls_done, bail_list, bail_count, use_list, list_off, opt.trace, opt.trace_stride, opt.memo, opt.force_serial, opt.cost, opt.enable);
+  return cudaLaunchKernelEx(&cfg, k_track<C>, bins, w, h, d_slots, mh, ch, state, n_calls, d_objs, d_win, flag, stats,
+                            order, list_off, opt.trace, opt.trace_stride, opt.memo, opt.force_serial, opt.cost, opt.enable);
 }
 
-// cluster size x CTA size chosen at run time
-template <int NT>
-cudaError_t launch_track_nt(int c, cudaStream_t st, int n, const uint16_t *bins, int w, int h, const int32_t *d_slots,
-                            const uint32_t *mh, const uint32_t *ch, TrackState *state, int n_calls, int32_t *d_objs,
-                            int32_t *d_win, int32_t *flag, unsigned long long *stats, int32_t *calls_done, int32_t *list,
-                            int32_t *count, int use_list, int list_off, TrackOpts opt) {
+// cluster size chosen at run time: 2, 4 or 8 CTAs per stream (any other value: 8)
+cudaError_t launch_track_cluster(int c, cudaStream_t st, int n, const uint16_t *bins, int w, int h, const int32_t *d_slots,
+                                 const uint32_t *mh, const uint32_t *ch, TrackState *state, int n_calls, int32_t *d_objs,
+                                 int32_t *d_win, int32_t *flag, unsigned long long *stats, const int32_t *order,
+                                 int list_off, TrackOpts opt) {
   switch (c) {
-    case 1: return launch_track_c<1, NT>(st, n, bins, w, h, d_slots, mh, ch, state, n_calls, d_objs, d_win, flag, stats, 0, calls_done, list, count, use_list, list_off, opt);
-    case 2: return launch_track_c<2, NT>(st, n, bins, w, h, d_slots, mh, ch, state, n_calls, d_objs, d_win, flag, stats, 0, calls_done, list, count, use_list, list_off, opt);
-    case 4: return launch_track_c<4, NT>(st, n, bins, w, h, d_slots, mh, ch, state, n_calls, d_objs, d_win, flag, stats, 0, calls_done, list, count, use_list, list_off, opt);
-    case 16: {
-      static bool allowed = false;   // clusters of 16 are a non-portable size: opt in once per instantiation
-      if (!allowed) {
-        cudaError_t e = cudaFuncSetAttribute(k_track<16, NT>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-        if (e != cudaSuccess) return e;
-        allowed = true;
-      }
-      return launch_track_c<16, NT>(st, n, bins, w, h, d_slots, mh, ch, state, n_calls, d_objs, d_win, flag, stats, 0, calls_done, list, count, use_list, list_off, opt);
-    }
-    default: return launch_track_c<8, NT>(st, n, bins, w, h, d_slots, mh, ch, state, n_calls, d_objs, d_win, flag, stats, 0, calls_done, list, count, use_list, list_off, opt);
+    case 2: return launch_track_c<2>(st, n, bins, w, h, d_slots, mh, ch, state, n_calls, d_objs, d_win, flag, stats, order, list_off, opt);
+    case 4: return launch_track_c<4>(st, n, bins, w, h, d_slots, mh, ch, state, n_calls, d_objs, d_win, flag, stats, order, list_off, opt);
+    default: return launch_track_c<8>(st, n, bins, w, h, d_slots, mh, ch, state, n_calls, d_objs, d_win, flag, stats, order, list_off, opt);
   }
-}
-cudaError_t launch_track_any(int c, int nt, cudaStream_t st, int n, const uint16_t *bins, int w, int h, const int32_t *d_slots,
-                             const uint32_t *mh, const uint32_t *ch, TrackState *state, int n_calls, int32_t *d_objs,
-                             int32_t *d_win, int32_t *flag, unsigned long long *stats, int32_t *calls_done, int32_t *list,
-                             int32_t *count, int use_list, int list_off, TrackOpts opt) {
-  if (nt == 512)
-    return launch_track_nt<512>(c, st, n, bins, w, h, d_slots, mh, ch, state, n_calls, d_objs, d_win, flag, stats, calls_done, list, count, use_list, list_off, opt);
-  if (nt == 128)
-    return launch_track_nt<128>(c, st, n, bins, w, h, d_slots, mh, ch, state, n_calls, d_objs, d_win, flag, stats, calls_done, list, count, use_list, list_off, opt);
-  return launch_track_nt<256>(c, st, n, bins, w, h, d_slots, mh, ch, state, n_calls, d_objs, d_win, flag, stats, calls_done, list, count, use_list, list_off, opt);
 }
 
 int launch_track(ht_ctx *ctx, int n, int f0, const uint16_t *bins, int w, int h, const int32_t *d_slots, const uint32_t *mh,
@@ -788,93 +747,65 @@ int launch_track(ht_ctx *ctx, int n, int f0, const uint16_t *bins, int w, int h,
                       // (the kernel indexes both areas with the stream number relative to f0)
                       4 * (size_t)ctx->cfg.max_frames - 4 * (size_t)f0 + 8 * (size_t)f0,
                       ctx->track_memo ? 1 : 0, (ctx->force_ties & 4) ? 1 : 0, ctx->d_track_cost.as<int32_t>(), enable};
-  // per-chunk scheduling scratch: [calls_done | area n][bail_list | order n][bail_count 1]
-  int32_t *calls_done = ctx->d_sched.as<int32_t>() + (size_t)f0;
-  int32_t *bail_list = ctx->d_sched.as<int32_t>() + (size_t)ctx->cfg.max_frames + f0;
-  int32_t *bail_count = ctx->d_sched.as<int32_t>() + 2 * (size_t)ctx->cfg.max_frames + (ctx->sched_seq++ & 63);
+  // per-chunk launch-order scratch: [area n][order n]
+  int32_t *area = ctx->d_sched.as<int32_t>() + (size_t)f0;
+  int32_t *order = ctx->d_sched.as<int32_t>() + (size_t)ctx->cfg.max_frames + f0;
   cudaError_t e = cudaSuccess;
-  if (ctx->track_bail_area > 0) {
-    // two-phase (HT_TRACK_BAIL=<px>): measured 8.1-8.9 ms per 1024x30 calls vs 7.2 ms for the single-phase cluster of 4
-    e = cudaMemsetAsync(bail_count, 0, sizeof(int32_t), st);
-    if (e != cudaSuccess) return ctx->fail(HT_ERR_CUDA, "memset: %s", cudaGetErrorString(e));
-    e = launch_track_c<1>(st, n, bins, w, h, d_slots, mh, ch, state, n_calls, d_objs, d_win, flag, stats, ctx->track_bail_area,
-                          calls_done, bail_list, bail_count, 0, 0, opt);
-    if (e == cudaSuccess)
-      e = launch_track_c<8>(st, n, bins, w, h, d_slots, mh, ch, state, n_calls, d_objs, d_win, flag, stats, 0, calls_done,
-                            bail_list, bail_count, 1, 0, opt);
-    ctx->launches += 2;
+  // few streams -> 8 CTAs per stream (latency of one stream); many streams -> 2 (more streams resident).
+  // measured on 1024 streams x 30 calls in index order: 1 CTA 9.7 ms, 2 CTAs 6.1 ms, 4 CTAs 6.2 ms, 8 CTAs 10.1 ms
+  int c = ctx->track_cluster;
+  if (c <= 0) c = (n >= 256) ? 2 : (n >= 32 ? 4 : 8);
+  const bool lpt = ctx->track_lpt && n >= 128;     // below that every stream is resident from the start
+  if (!lpt) {
+    e = launch_track_cluster(c, st, n, bins, w, h, d_slots, mh, ch, state, n_calls, d_objs, d_win, flag, stats, nullptr, 0, opt);
+    ++ctx->launches;
   } else {
-    // few streams -> 8 CTAs per stream (latency of one stream); many streams -> 2 (more streams resident).
-    // measured on 1024 streams x 30 calls in index order: 1 CTA 9.7 ms, 2 CTAs 6.1 ms, 4 CTAs 6.2 ms, 8 CTAs 10.1 ms
-    int c = ctx->track_cluster;
-    if (c <= 0) c = (n >= 256) ? 2 : (n >= 32 ? 4 : 8);
-    const int nt = ctx->track_nt;
-    const bool lpt = ctx->track_lpt && n >= 128;     // below that every stream is resident from the start
-    if (!lpt) {
-      e = launch_track_any(c, nt, st, n, bins, w, h, d_slots, mh, ch, state, n_calls, d_objs, d_win, flag, stats, calls_done,
-                           bail_list, bail_count, 0, 0, opt);
-      ++ctx->launches;
-    } else {
-      // longest chain first: order the streams by search-window area (k_track_area / k_track_rank); optionally the
-      // n / track_heavy_div largest get a cluster of 8 on a second stream, concurrently with the others
-      k_track_area<<<(n + 255) / 256, 256, 0, st>>>(state, d_slots, n, ctx->track_history ? ctx->d_track_cost.as<int32_t>() : nullptr, calls_done);
-      k_track_rank<<<(n + 255) / 256, 256, 0, st>>>(calls_done, n, bail_list);
-      ctx->launches += 2;
-      // Tiers by cost rank, each on its own stream so that they run concurrently, costliest first:
-      //   the costliest n / heavy_div streams on clusters of 8 (long chains over large windows: shorten every pass),
-      //   the next n / mid_div on clusters of 4, the cheapest n / light_div on single CTAs (small windows, few passes:
-      //   no cluster barrier at all, and half the CTA slots), the rest on clusters of `c` (2).
-      struct Tier { int count, cluster, threads, side; };   // side >= 0: ctx->tier_stream[side]; -1: the context's stream
-      Tier tiers[4];
-      int n_tiers = 0, left = n;
-      auto take = [&](int div, int cl, int threads, int side) {
-        const int k = (div > 0) ? std::min(left, n / div) : 0;
-        if (k > 0) { tiers[n_tiers++] = Tier{k, cl, threads, side}; left -= k; }
-        return k;
-      };
-      take(ctx->track_heavy_div, ctx->track_heavy_cluster, 256, 0);
-      take(ctx->track_mid_div, ctx->track_mid_cluster, 256, 1);
-      const int n_light = (ctx->track_light_div > 0) ? std::min(left, (int)((double)n / ctx->track_light_div)) : 0;
-      // Round 2, call 8 timeline: with the default tier on the context's own stream (no event wait) its 1,888 CTAs
-      // reached the GPU first and filled every slot with ITS costliest streams; the heavy and middle tiers - the
-      // longest chains of the launch - started 1.4 ms late and the launch ended at 1.4 + 2.3 ms.  Now every tier sits
-      // on a side stream behind the same event, submitted costliest tier first, and the side streams carry
-      // descending priorities (heavy > mid > rest > light), so a free slot always goes to the longest pending chain.
-      const bool rest_side = ctx->track_prio != 0 && (ctx->track_heavy_div > 0 || ctx->track_mid_div > 0);
-      if (left - n_light > 0) tiers[n_tiers++] = Tier{left - n_light, c, nt, rest_side ? 3 : -1};
-      if (n_light > 0) tiers[n_tiers++] = Tier{n_light, 1, ctx->track_light_nt, 2};
-      if (n_tiers > 1) {
-        int prio_least = 0, prio_greatest = 0;
-        CK(cudaDeviceGetStreamPriorityRange(&prio_least, &prio_greatest));   // numerically lower = more urgent
-        int prio_top = prio_greatest;
-        if (ctx->pipeline && ctx->pipe_bg) {   // background mode: every tier below the context's own stream
-          int pm = 0;
-          CK(cudaStreamGetPriority(ctx->main_stream ? ctx->main_stream : ctx->stream, &pm));
-          prio_top = std::min(prio_least, pm + 1);
+    // longest chain first: order the streams by their expected cost (k_track_area / k_track_rank)
+    k_track_area<<<(n + 255) / 256, 256, 0, st>>>(state, d_slots, n, ctx->d_track_cost.as<int32_t>(), area);
+    k_track_rank<<<(n + 255) / 256, 256, 0, st>>>(area, n, order);
+    ctx->launches += 2;
+    // Tiers by cost rank, each on its own stream so that they run concurrently, costliest first:
+    //   the costliest n / heavy_div streams on clusters of 8 (long chains over large windows: shorten every pass),
+    //   the next n / mid_div on clusters of 4, the rest on clusters of `c` (2).
+    struct Tier { int count, cluster, side; };   // side >= 0: ctx->tier_stream[side]; -1: the context's stream
+    Tier tiers[3];
+    int n_tiers = 0, left = n;
+    auto take = [&](int div, int cl, int side) {
+      const int k = (div > 0) ? std::min(left, n / div) : 0;
+      if (k > 0) { tiers[n_tiers++] = Tier{k, cl, side}; left -= k; }
+    };
+    take(ctx->track_heavy_div, ctx->track_heavy_cluster, 0);
+    take(ctx->track_mid_div, ctx->track_mid_cluster, 1);
+    // Round 2, call 8 timeline: with the default tier on the context's own stream (no event wait) its 1,888 CTAs
+    // reached the GPU first and filled every slot with ITS costliest streams; the heavy and middle tiers - the
+    // longest chains of the launch - started 1.4 ms late and the launch ended at 1.4 + 2.3 ms.  Now every tier sits
+    // on a side stream behind the same event, submitted costliest tier first, and the side streams carry
+    // descending priorities (heavy > mid > rest), so a free slot always goes to the longest pending chain.
+    const bool rest_side = ctx->track_heavy_div > 0 || ctx->track_mid_div > 0;
+    if (left > 0) tiers[n_tiers++] = Tier{left, c, rest_side ? 2 : -1};
+    if (n_tiers > 1) {
+      int prio_least = 0, prio_greatest = 0;
+      CK(cudaDeviceGetStreamPriorityRange(&prio_least, &prio_greatest));   // numerically lower = more urgent
+      for (int t = 0; t < 3; ++t)
+        if (!ctx->tier_stream[t]) {
+          CK(cudaStreamCreateWithPriority(&ctx->tier_stream[t], cudaStreamNonBlocking, std::min(prio_least, prio_greatest + t)));
+          CK(cudaEventCreateWithFlags(&ctx->tier_done[t], cudaEventDisableTiming));
         }
-        for (int t = 0; t < 4; ++t)
-          if (!ctx->tier_stream[t]) {
-            const int rank = (t == 0) ? 0 : (t == 1 ? 1 : (t == 3 ? 2 : 3));   // heavy, mid, rest, light
-            const int prio = ctx->track_prio ? std::min(prio_least, prio_top + rank) : prio_least;
-            CK(cudaStreamCreateWithPriority(&ctx->tier_stream[t], cudaStreamNonBlocking, prio));
-            CK(cudaEventCreateWithFlags(&ctx->tier_done[t], cudaEventDisableTiming));
-          }
-        if (!ctx->sched_ready) CK(cudaEventCreateWithFlags(&ctx->sched_ready, cudaEventDisableTiming));
-        CK(cudaEventRecord(ctx->sched_ready, st));
-      }
-      int off = 0;
-      for (int t = 0; t < n_tiers && e == cudaSuccess; ++t) {
-        cudaStream_t ts = tiers[t].side >= 0 ? ctx->tier_stream[tiers[t].side] : st;
-        if (tiers[t].side >= 0) CK(cudaStreamWaitEvent(ts, ctx->sched_ready, 0));
-        e = launch_track_any(tiers[t].cluster, tiers[t].threads, ts, tiers[t].count, bins, w, h, d_slots, mh, ch, state, n_calls,
-                             d_objs, d_win, flag, stats, calls_done, bail_list, bail_count, 2, off, opt);
-        ++ctx->launches;
-        if (tiers[t].side >= 0) CK(cudaEventRecord(ctx->tier_done[tiers[t].side], ts));
-        off += tiers[t].count;
-      }
-      for (int t = 0; t < n_tiers; ++t)
-        if (tiers[t].side >= 0) CK(cudaStreamWaitEvent(st, ctx->tier_done[tiers[t].side], 0));
+      if (!ctx->sched_ready) CK(cudaEventCreateWithFlags(&ctx->sched_ready, cudaEventDisableTiming));
+      CK(cudaEventRecord(ctx->sched_ready, st));
     }
+    int off = 0;
+    for (int t = 0; t < n_tiers && e == cudaSuccess; ++t) {
+      cudaStream_t ts = tiers[t].side >= 0 ? ctx->tier_stream[tiers[t].side] : st;
+      if (tiers[t].side >= 0) CK(cudaStreamWaitEvent(ts, ctx->sched_ready, 0));
+      e = launch_track_cluster(tiers[t].cluster, ts, tiers[t].count, bins, w, h, d_slots, mh, ch, state, n_calls, d_objs, d_win,
+                               flag, stats, order, off, opt);
+      ++ctx->launches;
+      if (tiers[t].side >= 0) CK(cudaEventRecord(ctx->tier_done[tiers[t].side], ts));
+      off += tiers[t].count;
+    }
+    for (int t = 0; t < n_tiers; ++t)
+      if (tiers[t].side >= 0) CK(cudaStreamWaitEvent(st, ctx->tier_done[tiers[t].side], 0));
   }
   if (e != cudaSuccess) return ctx->fail(HT_ERR_CUDA, "k_track launch: %s", cudaGetErrorString(e));
   return HT_OK;
@@ -903,14 +834,10 @@ int track_init_common(ht_ctx *ctx, const int32_t *slots, int n, const uint8_t *d
 // Shared memory of one k_cascade CTA: the staged tile and three sets of per-class survivor bit masks.
 constexpr size_t CASC_SMEM = (size_t)TILE_WORDS * 4 + 3 * (size_t)MASK_WORDS * 32 * sizeof(uint32_t);
 constexpr size_t GRAY_HIST_SMEM = 2 * 4096 * sizeof(uint32_t);   // two frames per word, 16-bit counters
-// (ht_set_pipeline, background mode) dynamic shared memory that lets exactly THREE k_cascade CTAs share an SM and leaves
-// room for one k_track CTA (35.5 KB static): 4 x (57,600 + 1 KB reserved) > 228 KB, 3 x 58,624 + 36,480 <= 233,472
-constexpr size_t CASC_SMEM_BG = 57600;
-static_assert(CASC_SMEM <= CASC_SMEM_BG || HT_TILE_TH > 8, "background padding assumes the 32x8 tile");
 
 int set_kernel_attributes(ht_ctx *ctx) {
-  CK(cudaFuncSetAttribute(k_cascade<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max(CASC_SMEM, CASC_SMEM_BG)));
-  CK(cudaFuncSetAttribute(k_cascade<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max(CASC_SMEM, CASC_SMEM_BG)));
+  CK(cudaFuncSetAttribute(k_cascade<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CASC_SMEM));
+  CK(cudaFuncSetAttribute(k_cascade<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CASC_SMEM));
   CK(cudaFuncSetAttribute(k_cascade<true>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
   CK(cudaFuncSetAttribute(k_cascade<false>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
   CK(cudaFuncSetAttribute(k_gray<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GRAY_HIST_SMEM));
@@ -1065,9 +992,7 @@ int run_detect(ht_ctx *ctx, Plan *P, const uint8_t *d_rgba_batch, int f0, int n,
     if (!P->casc_tiles.empty()) {
       ctx->prof_begin(HT_PROF_CASCADE);
       auto kern = ctx->hc.fast ? k_cascade<true> : k_cascade<false>;
-      // background mode: while the previous call's tracking is in flight, three cascade CTAs per SM instead of four
-      const size_t casc_smem = (before_group && ctx->pipe_bg) ? std::max(CASC_SMEM, CASC_SMEM_BG) : CASC_SMEM;
-      kern<<<dim3((unsigned)P->casc_tiles.size(), quads), CASCADE_THREADS, casc_smem, st>>>(
+      kern<<<dim3((unsigned)P->casc_tiles.size(), quads), CASCADE_THREADS, CASC_SMEM, st>>>(
           P->dplan, ctx->d_casc.as<LateFeat>(), ctx->d_casc.as<LateFeat>() + ctx->hc.n_sched, ctx->d_late_chunk0.as<int32_t>(),
           (ctx->use_tma && ctx->d_tmaps.p) ? ctx->d_tmaps.as<uint8_t>() + (piped ? (size_t)(wi & 1) : 0) * P->scales.size() * 128 : nullptr, 0,
           arena, P->arena_stride, nw,
@@ -1198,25 +1123,15 @@ int ht_create(ht_ctx **out, const ht_config *cfg, const void *cascade_blob, size
     c->own_stream = true;
   }
   if (const char *tc = getenv("HT_TRACK_CLUSTER")) c->track_cluster = atoi(tc);
-  if (const char *ba = getenv("HT_TRACK_BAIL")) c->track_bail_area = atoi(ba);
   if (const char *dp = getenv("HT_DETECT_PIPE")) c->detect_pipe = std::max(0, atoi(dp));
   if (const char *tm2 = getenv("HT_TRACK_MEMO")) c->track_memo = atoi(tm2) != 0;
   if (const char *tt = getenv("HT_TRACK_TRACE")) c->track_trace = atoi(tt) != 0;
-  if (const char *tn = getenv("HT_TRACK_NT")) c->track_nt = (atoi(tn) == 128) ? 128 : (atoi(tn) == 512 ? 512 : 256);
   if (const char *tl = getenv("HT_TRACK_LPT")) c->track_lpt = atoi(tl) != 0;
-  if (const char *thi = getenv("HT_TRACK_HISTORY")) c->track_history = atoi(thi) != 0;
   if (const char *th = getenv("HT_TRACK_HEAVY")) {
     c->track_heavy_div = std::max(0, atoi(th));
     if (const char *comma = strchr(th, ',')) {
       const int hc = atoi(comma + 1);
-      if (hc == 1 || hc == 2 || hc == 4 || hc == 8 || hc == 16) c->track_heavy_cluster = hc;
-    }
-  }
-  if (const char *tli = getenv("HT_TRACK_LIGHT")) {
-    c->track_light_div = std::max(0.0, atof(tli));
-    if (const char *comma = strchr(tli, ',')) {
-      const int ln = atoi(comma + 1);
-      if (ln == 128 || ln == 256 || ln == 512) c->track_light_nt = ln;
+      if (hc == 2 || hc == 4 || hc == 8) c->track_heavy_cluster = hc;
     }
   }
   if (const char *tmid = getenv("HT_TRACK_MID")) {
@@ -1229,12 +1144,9 @@ int ht_create(ht_ctx **out, const ht_config *cfg, const void *cascade_blob, size
   if (const char *wv = getenv("HT_WAVE")) c->wave_frames = std::max(4, atoi(wv));
   if (const char *wm = getenv("HT_WAVE_MB")) c->wave_mb = std::max(1, atoi(wm));
   if (const char *tm = getenv("HT_TMA")) c->use_tma = atoi(tm) != 0;
-  if (HT_UNIBASE) c->use_tma = false;       // super-row tiles: a dense TMA box cannot be written into them
   if (const char *ov = getenv("HT_OVERLAP")) { c->overlap_track = atoi(ov) != 0 ? 1 : 0; c->overlap_parts = atoi(ov); }
   if (const char *hc2 = getenv("HT_H2D_CHUNK")) c->h2d_chunk = std::max(1, atoi(hc2));
   if (const char *pl = getenv("HT_PIPELINE")) c->pipeline = atoi(pl) != 0 ? 1 : 0;
-  if (const char *bg = getenv("HT_PIPE_BG")) c->pipe_bg = atoi(bg) != 0 ? 1 : 0;
-  if (const char *tp = getenv("HT_TRACK_PRIO")) c->track_prio = atoi(tp) != 0 ? 1 : 0;
   if (const char *tk = getenv("HT_TRACK_MASK")) {   // HT_TRACK_MASK=<min n_calls>[,<min frames swept>]  (0: off / 0: every stream)
     c->track_mask_min = std::max(0, atoi(tk));
     if (const char *comma = strchr(tk, ',')) c->track_mask_frames = std::max(0, atoi(comma + 1));
@@ -1285,13 +1197,11 @@ void ht_destroy(ht_ctx *ctx) {
   if (ctx->pipe_stream) cudaStreamDestroy(ctx->pipe_stream);
   if (ctx->pipe_start) cudaEventDestroy(ctx->pipe_start);
   for (cudaEvent_t e : ctx->pipe_events) if (e) cudaEventDestroy(e);
-  if (ctx->sched_stream) cudaStreamDestroy(ctx->sched_stream);
-  for (int t = 0; t < 4; ++t) {
+  for (int t = 0; t < 3; ++t) {
     if (ctx->tier_stream[t]) cudaStreamDestroy(ctx->tier_stream[t]);
     if (ctx->tier_done[t]) cudaEventDestroy(ctx->tier_done[t]);
   }
   if (ctx->sched_ready) cudaEventDestroy(ctx->sched_ready);
-  if (ctx->sched_done) cudaEventDestroy(ctx->sched_done);
   if (ctx->aux_stream) cudaStreamDestroy(ctx->aux_stream);
   if (ctx->aux_done) cudaEventDestroy(ctx->aux_done);
   if (ctx->pipe_detect_done) cudaEventDestroy(ctx->pipe_detect_done);
@@ -1475,11 +1385,9 @@ int ht_detect_track(ht_ctx *ctx, const uint8_t *rgba, int n, int w, int h, int i
       CK(ctx->bins.reserve(2 * plane_elems * sizeof(uint16_t)));
     }
     if (!ctx->aux_stream) {
-      int prio_least = 0, prio_greatest = 0, aux_prio = 0;
+      int prio_least = 0, prio_greatest = 0;
       CK(cudaDeviceGetStreamPriorityRange(&prio_least, &prio_greatest));
-      aux_prio = prio_greatest;
-      if (ctx->pipe_bg) { int pm = 0; CK(cudaStreamGetPriority(st, &pm)); aux_prio = std::min(prio_least, pm + 1); }
-      CK(cudaStreamCreateWithPriority(&ctx->aux_stream, cudaStreamNonBlocking, aux_prio));
+      CK(cudaStreamCreateWithPriority(&ctx->aux_stream, cudaStreamNonBlocking, prio_greatest));
       CK(cudaEventCreateWithFlags(&ctx->aux_done, cudaEventDisableTiming));
       for (int i = 0; i < 4; ++i) CK(cudaEventCreateWithFlags(&ctx->part_events[i], cudaEventDisableTiming));
     }
@@ -1494,12 +1402,10 @@ int ht_detect_track(ht_ctx *ctx, const uint8_t *rgba, int n, int w, int h, int i
     if (rc != HT_OK) return rc;
     CK(cudaEventRecord(ctx->pipe_detect_done, st));
     CK(cudaStreamWaitEvent(ctx->aux_stream, ctx->pipe_detect_done, 0));
-    ctx->main_stream = st;
     ctx->stream = ctx->aux_stream;
     rc = run_track_from_detect(ctx, rgba, w, h, 0, n, dr, out_counts, calc_angles, n_calls, out_found,
                                reinterpret_cast<int32_t *>(out_objs), reinterpret_cast<int32_t *>(out_windows));
     ctx->stream = st;
-    ctx->main_stream = nullptr;
     if (rc != HT_OK) return rc;
     CK(cudaEventRecord(ctx->aux_done, ctx->aux_stream));
     ctx->aux_pending = true;
@@ -2058,6 +1964,7 @@ extern "C" int ht_selftest_pyramid(int w, int h, int interval, const uint8_t *rg
 extern "C" int ht_selftest_cascade(const void *blob, size_t blob_len, int w, int h, int interval, const uint32_t *arena,
                                    int n_frames, int force_ties, int quad_stages, double *out /* [4][cap][4] x,y,width,conf */,
                                    int32_t *counts, int cap) {
+  if (quad_stages != HT_GEN_QUAD_STAGES) return -4;   // the dense group evaluates stages {0,1} in quad form, as k_cascade
   static HostCascade hc;   // (ConstCascade is 63 KB: keep it off the stack)
   std::string err;
   if (parse_cascade(blob, blob_len, hc, err) != HT_OK) { fprintf(stderr, "%s\n", err.c_str()); return -1; }
@@ -2121,11 +2028,10 @@ extern "C" int ht_selftest_cascade(const void *blob, size_t blob_len, int w, int
           a_lo = ((fmask & 1u) ? 0x8000u : 0u) | ((fmask & 4u) ? 0x80000000u : 0u);
           a_hi = ((fmask & 2u) ? 0x8000u : 0u) | ((fmask & 8u) ? 0x80000000u : 0u);
         }
-        for (int J = 0; J < quad_stages; ++J) {
+        for (int J = 0; J < HT_GEN_QUAD_STAGES; ++J) {
           uint32_t p_lo = 0, p_hi = 0, t_lo = 0, t_hi = 0;
           if (J == 0) gen_q_stage0(tA, tB, p_lo, p_hi, t_lo, t_hi);
-          else if (J == 1) gen_q_stage1(tA, tB, p_lo, p_hi, t_lo, t_hi);
-          else gen_q_stage2(tA, tB, p_lo, p_hi, t_lo, t_hi);
+          else gen_q_stage1(tA, tB, p_lo, p_hi, t_lo, t_hi);
           t_lo &= a_lo; t_hi &= a_hi;
           for (int f = 0; f < 4; ++f) {
             const uint32_t bit = (f & 2) ? 0x80000000u : 0x8000u;
@@ -2147,7 +2053,7 @@ extern "C" int ht_selftest_cascade(const void *blob, size_t blob_len, int w, int
         const uint8_t *tA, *tB;
         bases(e, tA, tB);
         bool alive = true;
-        for (int j = quad_stages; j < late_first && alive; ++j) {
+        for (int j = HT_GEN_QUAD_STAGES; j < late_first && alive; ++j) {
           int r = gen_stage(j, tA, tB);
           if (force_ties & 1) r = -1;
           if (r < 0) r = stage_pass_ordered(tA, tB, j) ? 1 : 0;

@@ -34,10 +34,7 @@ namespace ht {
 // (src/ccv.js:179-180,235-241).  2*P0 == P1 == P2 (mod 32), so bank(baseA) == bank(baseB) == (u + 12 v) & 31: the
 // "bank class" of the window.  Lane L only ever evaluates class-L windows -> conflict-free loads in every stage.
 constexpr int TW = 32;
-#ifndef HT_TILE_TH
-#define HT_TILE_TH 8
-#endif
-constexpr int TH = HT_TILE_TH;                // quarter-res rows of a tile (8: four CTAs per SM, 16: two)
+constexpr int TH = 8;                         // quarter-res rows of a tile
 constexpr int NV = 2 * TH;                    // v values of a tile
 constexpr int L0_COLS = 4 * TW + 22;          // 150 level-0 columns
 constexpr int L0_ROWS = 4 * TH + 22;
@@ -49,29 +46,17 @@ constexpr int P1 = 76;
 constexpr int L2_ROWS = TH + 5;               // per copy
 constexpr int L2_COLS = TW + 5;               // 37 per copy
 constexpr int P2 = 76;
-// Two shared-memory arrangements of the three levels:
-//   HT_UNIBASE == 0 (default): three separate blocks (level 1 a dense box that the TMA engine can write), two per-window bases.
-//   HT_UNIBASE == 1: "super-rows" (measured 1.6 % SLOWER: 6.41 vs 6.31 ms, level 1 loses its TMA staging) - for every v one row [level-0 row 2v | level-0 row 2v+1 | level-1 row v |
-//     level-2 row v] of SR words.  Every point of every level is then  base + constant  for ONE base  v * SR + u:
-//     the late stages form an address with one add instead of select + add, and a window carries one base register.
-#ifndef HT_UNIBASE
-#define HT_UNIBASE 0
-#endif
-constexpr int W1 = (L0_ROWS * P0 + 31) / 32 * 32;   // (separate blocks) 128-byte aligned: the level-1 box can be written by TMA
+// The three levels are separate blocks (level 1 a dense box that the TMA engine can write), with two per-window bases.
+constexpr int W1 = (L0_ROWS * P0 + 31) / 32 * 32;   // 128-byte aligned: the level-1 box can be written by TMA
 constexpr int W2 = W1 + L1_ROWS * P1;
-constexpr int SR = 2 * P0 + P1 + P2;                // (super-rows) 452 words = 113 x 16 bytes
-static_assert(L0_ROWS == 2 * L1_ROWS && 2 * L2_ROWS <= L1_ROWS, "super-rows: level 0 has two rows per v, levels 1 and 2 one");
-static_assert((2 * P0) % 4 == 0 && (2 * P0 + P1) % 4 == 0 && SR % 4 == 0, "16-byte aligned level blocks inside a super-row");
-constexpr int TILE_WORDS = HT_UNIBASE ? L1_ROWS * SR : W2 + 2 * L2_ROWS * P2;
+constexpr int TILE_WORDS = W2 + 2 * L2_ROWS * P2;
 // word of level-0 pixel (row r, column X), level-1 pixel (r, c), interleaved level-2 entry (row rr = 2Y+dy, column c2 = 2X+dx)
-__host__ __device__ constexpr int tile_l0(int r, int X) {
-  return HT_UNIBASE ? (r >> 1) * SR + (r & 1) * P0 + (X & 1) * H0 + (X >> 1) : r * P0 + (X & 1) * H0 + (X >> 1);
-}
-__host__ __device__ constexpr int tile_l1(int r, int c) { return HT_UNIBASE ? r * SR + 2 * P0 + c : W1 + r * P1 + c; }
-__host__ __device__ constexpr int tile_l2(int rr, int c2) { return HT_UNIBASE ? rr * SR + 2 * P0 + P1 + c2 : W2 + rr * P2 + c2; }
+__host__ __device__ constexpr int tile_l0(int r, int X) { return r * P0 + (X & 1) * H0 + (X >> 1); }
+__host__ __device__ constexpr int tile_l1(int r, int c) { return W1 + r * P1 + c; }
+__host__ __device__ constexpr int tile_l2(int rr, int c2) { return W2 + rr * P2 + c2; }
 // words per unit of v of the two window bases: baseA = v * VA + u (level 0), baseB = v * VB + u (levels 1, 2)
-constexpr int VA = HT_UNIBASE ? SR : 2 * P0;
-constexpr int VB = HT_UNIBASE ? SR : P1;
+constexpr int VA = 2 * P0;
+constexpr int VB = P1;
 static_assert((VA - VB) % 32 == 0 && P1 == P2, "bank classes of the two bases must coincide");
 static_assert(2 * L2_COLS <= P2 && L1_COLS <= P1, "tile pitches");
 constexpr int BANK_K = VA % 32;               // bank(baseA) = bank(baseB) = (u + BANK_K * v) & 31
@@ -81,11 +66,9 @@ constexpr int NWIN = TW * TH * 4 * 4;         // windows per tile (4 phases x 4 
 // + 32 uh, each in 4 frames -> bit 8 v + 4 uh + f of the class's mask (NV / 4 words).  masks[word][class].
 constexpr int MASK_WORDS = NV / 4;
 static_assert(NV % 4 == 0, "TH must be even");
-#ifndef HT_CASC_THREADS
-#define HT_CASC_THREADS 256
-#endif
-constexpr int CASCADE_THREADS = HT_CASC_THREADS;
+constexpr int CASCADE_THREADS = 256;
 constexpr int CASCADE_WARPS = CASCADE_THREADS / 32;
+constexpr int CASCADE_MIN_BLOCKS = 4;         // resident k_cascade CTAs per SM the register allocation aims at
 // shared-memory WORD offset of point (z, x, y) of the 24x24 window relative to baseA (z == 0) or baseB (z > 0)
 __host__ __device__ constexpr int point_word(int z, int x, int y) {
   return z == 0 ? tile_l0(y, x) : z == 1 ? tile_l1(y, x) : tile_l2(2 * y, 2 * x);
@@ -94,12 +77,8 @@ __host__ __device__ constexpr int bank_class(int u, int v) { return (u + BANK_K 
 // the window of class c at (v, uh)
 __host__ __device__ constexpr int class_u(int c, int v, int uh) { return ((c - BANK_K * v) & 31) + 32 * uh; }
 
-// survivor groups of the generated cascade after the dense group {0,1}: 0: {2} {3} {4,5} {6,7}; 1: {2} {3} {4} {5} {6,7};
-// 2: {2} {3} {4} {5} {6} {7}.  A split costs a CTA barrier and repacks the survivors (tools/early_exit_model.py: 9 live
-// lanes per warp iteration in stage 5 and 6 in stage 7 with the groups of 0).
-#ifndef HT_GROUP_SPLIT
-#define HT_GROUP_SPLIT 0
-#endif
+// survivor groups of the generated cascade after the dense group {0,1}: {2} {3} {4,5} {6,7}.  A split costs a CTA barrier
+// and repacks the survivors (tools/early_exit_model.py: 9 live lanes per warp iteration in stage 5 and 6 in stage 7).
 constexpr int MAX_STAGES = 64;
 constexpr int MAX_GROUPS = 16;
 
@@ -194,7 +173,7 @@ struct alignas(16) LateFeat {
 static_assert(sizeof(LateFeat) == 48, "LateFeat is three 16-byte loads");
 constexpr uint32_t LATE_UNUSED = 0xFFFFFFFFu;
 // ConstCascade::off encoding (u16: word offset, bit 15 = baseB, 0xFFFF = unused) <-> LateFeat::off encoding
-__host__ __device__ constexpr uint32_t late_encode(uint16_t o) {   // (HT_UNIBASE: bit 15 / bit 31 are never set)
+__host__ __device__ constexpr uint32_t late_encode(uint16_t o) {
   return o == 0xFFFF ? LATE_UNUSED : (uint32_t)(o & 0x7fffu) * 4u | ((o & 0x8000u) ? 0x80000000u : 0u);
 }
 __host__ __device__ constexpr uint16_t late_decode(uint32_t o) {

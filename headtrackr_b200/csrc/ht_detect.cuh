@@ -399,9 +399,6 @@ __host__ __device__ __forceinline__ uint32_t lop3(uint32_t a, uint32_t b, uint32
 // stage decision as a truth table of the four "feature did not fire" bits: x3 ? B(x0,x1,x2) : A(x0,x1,x2)
 #define HT_LUT4(x0, x1, x2, x3, A, B) lop3<0xCA>(x3, lop3<B>(x0, x1, x2), lop3<A>(x0, x1, x2))
 #include "cascade_face_gen.inc"
-#ifndef HT_QUAD_STAGES
-#define HT_QUAD_STAGES 2   // stages the dense group evaluates in quad form (2: {0,1}; 3: {0,1,2})
-#endif
 #undef HT_GEN_FN
 #undef HT_PW
 #undef HT_MIN2
@@ -456,11 +453,7 @@ __device__ __forceinline__ bool feat_fires(unsigned sA, unsigned sBm, const uint
   unsigned vv[10];
 #pragma unroll
   for (int s = 0; s < 10; ++s) {
-#if HT_UNIBASE
-    const unsigned addr = sA + o[s];                                  // one base for all three levels
-#else
     const unsigned addr = ((int)o[s] < 0 ? sBm : sA) + o[s];
-#endif
     vv[s] = lds_u8_if(addr, o[s] != LATE_UNUSED, s < 5 ? 255u : 0u);   // unused slots: neutral element, no bank traffic
   }
   const unsigned pm = __vimin3_u32(__vimin3_u32(vv[0], vv[1], vv[2]), vv[3], vv[4]);
@@ -500,12 +493,6 @@ __device__ __forceinline__ void cp_async4(unsigned saddr, const void *g, bool va
 // Debug switches of the exactness fallbacks (ht_debug_set_exactness): bit 0 = treat every generated byte-stage
 // decision as a tie, bit 1 = treat every late-stage integer decision as a tie.  Ties are decided by the reference's
 // ordered fp64 adds, so results must not change (tests/test_gpu_quads.py).
-#ifndef HT_CASC_MINB
-#define HT_CASC_MINB (TH <= 8 ? 4 : (TH <= 12 ? 3 : 2))
-#endif
-#ifndef HT_CT_GROUPS
-#define HT_CT_GROUPS 1   // 1: the survivor groups of the generated cascade as four unrolled copies with constant stage bounds
-#endif
 // a compile-time int that converts to int in device code (std::integral_constant's conversion is a host function)
 template <int V>
 struct IntC {
@@ -545,7 +532,7 @@ __device__ __forceinline__ int nth_set_bit(const uint32_t *__restrict__ masks, i
 }
 
 template <bool FAST>
-__global__ void __launch_bounds__(CASCADE_THREADS, HT_CASC_MINB) k_cascade(DevPlan plan, const LateFeat *__restrict__ late,
+__global__ void __launch_bounds__(CASCADE_THREADS, CASCADE_MIN_BLOCKS) k_cascade(DevPlan plan, const LateFeat *__restrict__ late,
                                                                 const LateFeat *__restrict__ feat_orig,
                                                                 const int32_t *__restrict__ late_chunk0,
                                                                 const void *__restrict__ tmaps, int tma_quad0,
@@ -574,7 +561,7 @@ __global__ void __launch_bounds__(CASCADE_THREADS, HT_CASC_MINB) k_cascade(DevPl
   // Level 1 is a plain 2-D box of its plane (L1_ROWS x P1 words): when tensor maps are given it is staged by the
   // TMA engine - one elected thread issues cp.async.bulk.tensor (3-D map: column, row, frame quad; elements outside
   // the plane are zero-filled) completing on an mbarrier - while all threads scatter levels 0 and 2.
-  const bool use_tma = !HT_UNIBASE && tmaps != nullptr;   // a TMA box is dense: it cannot write into super-rows
+  const bool use_tma = tmaps != nullptr;
   if (use_tma) {
     const unsigned bar = (unsigned)__cvta_generic_to_shared(&tma_bar);
     if (tid == 0) {
@@ -584,7 +571,7 @@ __global__ void __launch_bounds__(CASCADE_THREADS, HT_CASC_MINB) k_cascade(DevPl
     __syncthreads();   // nobody may poll the barrier before it is initialised
     if (tid == 0) {
       asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"((unsigned)(L1_ROWS * P1 * 4)) : "memory");
-      const unsigned dst = (unsigned)__cvta_generic_to_shared(tile + W1);   // (separate-block layout only)
+      const unsigned dst = (unsigned)__cvta_generic_to_shared(tile + W1);
       const unsigned long long map = (unsigned long long)(reinterpret_cast<const uint8_t *>(tmaps) + 128 * (size_t)tl.scale);
       asm volatile(
           "cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
@@ -689,12 +676,10 @@ __global__ void __launch_bounds__(CASCADE_THREADS, HT_CASC_MINB) k_cascade(DevPl
   const int late_first = c_casc.group_first[c_casc.n_groups];
   const bool has_late = late_first < c_casc.n_stages;
   uint32_t *m_in = masks, *m_out = masks + MASK_WORDS * 32, *m_clr = masks + 2 * MASK_WORDS * 32;
-  int g = 0;
 
   // ---- dense group: every window of the tile.  A warp takes chunks of 4 (v, uh) units = 16 mask bits per lane ----
   {
-    constexpr int NQ = HT_QUAD_STAGES < HT_GEN_QUAD_STAGES ? HT_QUAD_STAGES : HT_GEN_QUAD_STAGES;
-    static_assert(NQ == 2 || NQ == 3, "the dense group is {0,1} or {0,1,2}");
+    static_assert(HT_GEN_QUAD_STAGES == 2, "the dense group is {0,1}");
     uint16_t *m16 = reinterpret_cast<uint16_t *>(m_in);
     for (int chunk = warp; chunk < NV / 2; chunk += CASCADE_WARPS) {
       uint32_t bits = 0;
@@ -712,7 +697,7 @@ __global__ void __launch_bounds__(CASCADE_THREADS, HT_CASC_MINB) k_cascade(DevPl
             a_hi = ((fmask & 2u) ? 0x8000u : 0u) | ((fmask & 8u) ? 0x80000000u : 0u);
           }
 #define HT_QSTAGE(J)                                                                                        \
-  if (NQ > J && __any_sync(0xffffffffu, (a_lo | a_hi) != 0u)) {                                              \
+  if (__any_sync(0xffffffffu, (a_lo | a_hi) != 0u)) {                                                        \
     uint32_t p_lo, p_hi, t_lo, t_hi;                                                                         \
     gen_q_stage##J(tA, tB, p_lo, p_hi, t_lo, t_hi);                                                          \
     t_lo &= a_lo; t_hi &= a_hi;                                                                              \
@@ -730,9 +715,6 @@ __global__ void __launch_bounds__(CASCADE_THREADS, HT_CASC_MINB) k_cascade(DevPl
   }
           HT_QSTAGE(0)
           HT_QSTAGE(1)
-#if HT_GEN_QUAD_STAGES >= 3
-          HT_QSTAGE(2)
-#endif
 #undef HT_QSTAGE
           m = ((a_lo >> 15) & 1u) | ((a_hi >> 14) & 2u) | ((a_lo >> 29) & 4u) | ((a_hi >> 28) & 8u);
         } else {
@@ -751,7 +733,6 @@ __global__ void __launch_bounds__(CASCADE_THREADS, HT_CASC_MINB) k_cascade(DevPl
       }
       m16[(((chunk >> 1) * 32 + lane) << 1) | (chunk & 1)] = (uint16_t)bits;
     }
-    g = FAST ? (NQ >= 3 ? 2 : 1) : 1;    // generated groups are {0,1} {2} {3} {4,5} {6,7}
   }
   __syncthreads();
 
@@ -814,29 +795,14 @@ __global__ void __launch_bounds__(CASCADE_THREADS, HT_CASC_MINB) k_cascade(DevPl
     return false;
   };
   if (FAST) {
-    // the generated groups {2} {3} {4,5} {6,7} (parse_cascade's cuts_fast; the dense group covered {0,1} or {0,1,2})
+    // the generated groups {2} {3} {4,5} {6,7} (parse_cascade's cuts_fast; the dense group covered {0,1})
     static_assert(HT_GEN_STAGES == 8, "compile-time groups assume 8 generated stages");
-#if HT_CT_GROUPS
-    if (g < 2 && run_group(IntC<2>{}, IntC<3>{}, false)) return;
+    if (run_group(IntC<2>{}, IntC<3>{}, false)) return;
     if (run_group(IntC<3>{}, IntC<4>{}, false)) return;
-#if HT_GROUP_SPLIT >= 1     // {4} {5}: one more barrier, survivors repacked between the two stages
-    if (run_group(IntC<4>{}, IntC<5>{}, false)) return;
-    if (run_group(IntC<5>{}, IntC<6>{}, false)) return;
-#else
     if (run_group(IntC<4>{}, IntC<6>{}, false)) return;
-#endif
-#if HT_GROUP_SPLIT >= 2     // {6} {7}
-    if (run_group(IntC<6>{}, IntC<7>{}, false)) return;
-    if (run_group(IntC<7>{}, IntC<8>{}, !has_late)) return;
-#else
     if (run_group(IntC<6>{}, IntC<8>{}, !has_late)) return;
-#endif
-#else   // one rolled copy of the group code (62 registers, no spills) - measured slower: 6.55 vs 6.28 ms per 1024 frames
-    for (; g < c_casc.n_groups; ++g)
-      if (run_group(c_casc.group_first[g], c_casc.group_first[g + 1], (g == c_casc.n_groups - 1) && !has_late)) return;
-#endif
   } else {
-    for (; g < c_casc.n_groups; ++g)
+    for (int g = 1; g < c_casc.n_groups; ++g)
       if (run_group(c_casc.group_first[g], c_casc.group_first[g + 1], (g == c_casc.n_groups - 1) && !has_late)) return;
   }
   if (!has_late) {

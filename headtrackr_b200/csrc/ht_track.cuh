@@ -229,14 +229,6 @@ __device__ __noinline__ Mom moments_serial(const uint16_t *__restrict__ px, int 
   return m;
 }
 
-#ifndef HT_TRACK_MBAR
-#define HT_TRACK_MBAR 0   // 1: partial moments travel with st.async + mbarrier (no cluster barrier, one CTA barrier per pass); measured 3.20 vs 3.15 ms - no gain, left off
-#endif
-__device__ __forceinline__ double warp_sum_all(double v) {   // every lane gets the total (same tree in every warp)
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
@@ -246,8 +238,9 @@ __device__ __forceinline__ double warp_sum(double v) {
 // One thread-block CLUSTER per slot: TRACK_CLUSTER CTAs split the rows of every window pass and
 // combine their partial moments through distributed shared memory.  Mean-shift is a serial chain
 // of passes per stream (up to 10 per track() call); spreading one pass over several SMs shortens
-// the chain of the streams with large windows, which otherwise set the kernel's duration.
-constexpr int TRACK_CLUSTER_MAX = 16;  // the cluster size is a launch-time choice (1, 2, 4, 8 or - non-portable - 16 CTAs per stream)
+// the chain of the streams with large windows, which otherwise set the kernel's duration.  The cluster size is a
+// launch-time choice: 2, 4 or 8 CTAs per stream.
+constexpr int TRACK_THREADS = 256;   // threads per k_track CTA
 
 // Longest-chain-first launch order.  A stream's mean-shift passes form a serial chain whose length grows with its
 // search window, and a launch holds only a few hundred streams at a time, so the streams with the largest windows
@@ -320,21 +313,15 @@ __device__ __forceinline__ void row_partial(const uint16_t *__restrict__ row, co
   }
 }
 
-template <int TRACK_CLUSTER, int NT>
-#ifndef HT_TRACK_MINB
-#define HT_TRACK_MINB 3   // resident 256-thread CTAs per SM the register allocation aims at (3: 80 registers, 4: 64)
-#endif
-__global__ void __launch_bounds__(NT, (NT >= 1024) ? 1 : (NT >= 512 ? 2 : (NT >= 256 ? HT_TRACK_MINB : 6)))
+// __launch_bounds__: three resident CTAs per SM (80 registers)
+template <int TRACK_CLUSTER>
+__global__ void __launch_bounds__(TRACK_THREADS, 3)
 k_track(const uint16_t *__restrict__ bins, int W, int H, const int32_t *__restrict__ slots,
         const uint32_t *__restrict__ model_hist, const uint32_t *__restrict__ cur_hist, TrackState *__restrict__ state,
         int n_calls, int32_t *__restrict__ out_objs /* 6 x i32 per frame */, int32_t *__restrict__ out_windows,
         int32_t *__restrict__ err_flag, unsigned long long *__restrict__ stats,
-        // two-phase scheduling: phase A (one CTA per stream) hands streams whose search window outgrows
-        // `bail_area` to phase B (a cluster per stream) through bail_list/calls_done
-        int bail_area, int32_t *__restrict__ calls_done, int32_t *__restrict__ bail_list,
-        int32_t *__restrict__ bail_count, int use_list,
-        // use_list == 2: the k-th cluster runs stream bail_list[list_off + k] (k_track_rank's order)
-        int list_off,
+        // order != NULL: the k-th cluster runs stream order[list_off + k] (k_track_rank's order); NULL: stream k
+        const int32_t *__restrict__ order, int list_off,
         // optional timeline (HT_TRACK_TRACE=1): per stream {globaltimer at start, at end, SM id, passes}
         unsigned long long *__restrict__ trace, size_t trace_stride,
         // memo != 0: moments are a pure function of (frame, weights, window) and all three are fixed for the calls of
@@ -350,21 +337,14 @@ k_track(const uint16_t *__restrict__ bins, int W, int H, const int32_t *__restri
   namespace cg = cooperative_groups;
   cg::cluster_group cluster = cg::this_cluster();
   __shared__ double wsm[4096 + 1];   // [4096] = +0.0: the weight of pixels outside the window
-  constexpr int NW = NT / 32;   // warps per CTA
+  constexpr int NW = TRACK_THREADS / 32;   // warps per CTA
   __shared__ double red[NW][6];
   // Every CTA of the cluster keeps its OWN copy of the reference's loop state and runs the scalar mean-shift step
   // redundantly (same inputs, same operations -> bit-identical windows), so a pass needs ONE cluster barrier - the
   // exchange of the partial moments - instead of two (round 1: partials to rank 0, barrier, rank 0 publishes the
   // next window, barrier).  cpart is double-buffered by pass parity: a CTA that is already exchanging pass p+1
   // cannot overwrite what a slower CTA still reads for pass p.
-  __shared__ double cpart[2][TRACK_CLUSTER_MAX][6];  // partial moments of every CTA of the cluster (written remotely)
-  // HT_TRACK_MBAR: every WARP of every CTA of the cluster sends its six partial sums straight into every CTA's wpart
-  // (st.async through distributed shared memory, completing bytes on the receiver's mbarrier); warp 0 of each CTA waits
-  // for 48 * C * NW bytes and adds them up in a fixed order.  Replaces red[] + __syncthreads + the cross-warp sum +
-  // cluster.sync (arrive.release / wait.acquire: 11 % of the kernel's samples plus 3.5 % for the CTA barrier).
-  constexpr bool MBAR = HT_TRACK_MBAR && TRACK_CLUSTER > 1 && TRACK_CLUSTER * NW <= 128;   // (12 KB of slots at most)
-  __shared__ double wpart[MBAR ? 2 : 1][MBAR ? TRACK_CLUSTER * NW : 1][6];
-  __shared__ __align__(8) unsigned long long mbar[2];
+  __shared__ double cpart[2][TRACK_CLUSTER][6];  // partial moments of every CTA of the cluster (written remotely)
   __shared__ int win[4];                          // wadx, wady, wadw, wadh of the next pass
   __shared__ int ctrl;                            // 0 = run another pass over win[], 1 = this stream is finished
   constexpr int MEMO_N = 8;
@@ -374,14 +354,7 @@ k_track(const uint16_t *__restrict__ bins, int W, int H, const int32_t *__restri
   __shared__ unsigned long long st_memo_sh;
   const int crank = (int)cluster.block_rank();
   int k = blockIdx.x / TRACK_CLUSTER;
-  int call0 = 0;
-  if (use_list == 2) {
-    k = bail_list[list_off + k];
-  } else if (use_list) {                          // phase B: k-th entry of the bail list (uniform over the cluster)
-    if (k >= *bail_count) return;
-    k = bail_list[k];
-    call0 = calls_done[k];
-  }
+  if (order) k = order[list_off + k];
   if (enable && !enable[k]) return;               // uniform over the cluster, before any cluster barrier
   const int slot = slots ? slots[k] : k;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -389,13 +362,12 @@ k_track(const uint16_t *__restrict__ bins, int W, int H, const int32_t *__restri
   const bool stepper = (tid == 0);                 // thread 0 of EVERY CTA runs the mean-shift step
   // The reference's loop state lives in shared memory: only the leader thread touches it after this point, and
   // keeping it out of registers leaves them to the pipelined pass loop.
-  struct Lead { TrackState s; unsigned long long st_pass, st_serial, st_px; int call, it, prevx, prevy; bool bailed; };
+  struct Lead { TrackState s; unsigned long long st_pass, st_serial, st_px; int call, it, prevx, prevy; };
   __shared__ Lead lead_sh;
   if (tid == 0) {
     lead_sh.s = state[slot];
     lead_sh.st_pass = lead_sh.st_serial = lead_sh.st_px = 0;
-    lead_sh.call = call0; lead_sh.it = 0; lead_sh.prevx = lead_sh.s.sx; lead_sh.prevy = lead_sh.s.sy;
-    lead_sh.bailed = false;
+    lead_sh.call = 0; lead_sh.it = 0; lead_sh.prevx = lead_sh.s.sx; lead_sh.prevy = lead_sh.s.sy;
     memo_next = 0; st_memo_sh = 0;
     for (int i = 0; i < MEMO_N; ++i) memo_tab[i].valid = 0;
   }
@@ -419,7 +391,7 @@ k_track(const uint16_t *__restrict__ bins, int W, int H, const int32_t *__restri
   // getWeights — src/camshift.js:314-330 (every CTA keeps its own copy)
   {
     const uint32_t *mh = model_hist + (size_t)slot * 4096, *ch = cur_hist + (size_t)k * 4096;
-    for (int i = tid; i < 4096; i += NT) {
+    for (int i = tid; i < 4096; i += TRACK_THREADS) {
       const uint32_t c = ch[i], m = mh[i];
       double p = 0.0;
       // (a bin absent from the model gives 0 / c = +0.0: no division for it - that is nearly all of the 4096 bins)
@@ -435,31 +407,21 @@ k_track(const uint16_t *__restrict__ bins, int W, int H, const int32_t *__restri
   // leader-only bookkeeping of the reference's loops (src/camshift.js:213-312)
   unsigned long long &st_pass = lead_sh.st_pass, &st_serial = lead_sh.st_serial, &st_px = lead_sh.st_px;
   int &call = lead_sh.call, &it = lead_sh.it, &prevx = lead_sh.prevx, &prevy = lead_sh.prevy;
-  bool &bailed = lead_sh.bailed;
   auto publish = [&](int done) {   // stepper: next window (or the finish flag) for this CTA
     const int w0 = max(s.sx, 0), w1 = max(s.sy, 0);                // :286-289
     const int w2 = min(w0 + s.sw, W), w3 = min(w1 + s.sh, H);
     win[0] = w0; win[1] = w1; win[2] = w2; win[3] = w3;
     ctrl = done;
   };
-  auto start_call = [&]() {        // leader: returns true when the stream stops here (all calls done, or bail-out)
+  auto start_call = [&]() {        // leader: returns true when all calls are done
     if (call >= n_calls) return true;
-    if (bail_area > 0 && (long long)s.sw * (long long)s.sh > (long long)bail_area) { bailed = true; return true; }
     it = 0; prevx = s.sx; prevy = s.sy;                            // :280-281
     return false;
   };
-  if (MBAR && tid == 0) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"((unsigned)__cvta_generic_to_shared(&mbar[0])));
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"((unsigned)__cvta_generic_to_shared(&mbar[1])));
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (TRACK_CLUSTER > 1) cluster.sync();  // every CTA is resident (and its mbarriers initialised) before the first remote access
+  if (TRACK_CLUSTER > 1) cluster.sync();  // every CTA is resident before the first remote access
   if (stepper) publish(start_call() ? 1 : 0);
   __syncthreads();
 
-#ifndef HT_TRACK_LOOP2
-#define HT_TRACK_LOOP2 0   // 1: column blocks outer, x factors per block, edge selects only where needed - measured 3.01 vs 2.97 ms: no gain, left off
-#endif
 #ifndef HT_TRACK_PASSTRACE
 #define HT_TRACK_PASSTRACE 0   // 1 (profiling build): the leader thread accumulates the clock cycles of each phase of a pass
 #endif
@@ -471,15 +433,11 @@ k_track(const uint16_t *__restrict__ bins, int W, int H, const int32_t *__restri
 #define HT_PT_MARK(i) do { } while (0)
 #endif
   constexpr int ROW_STRIDE = NW * TRACK_CLUSTER;
-  unsigned pass_no = 0;        // passes of this stream so far (uniform over the cluster): mbarrier / buffer parity
   while (!ctrl) {
     const int wx = win[0], wy = win[1], ww = win[2] - win[0], wh = win[3] - win[1];
 #if HT_TRACK_PASSTRACE
     if (trace && leader) pt_t = clock64();
 #endif
-    if (MBAR && tid == 0)      // arm this pass's mbarrier: one arrival (this one) + the bytes all warps of all CTAs will send
-      asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"((unsigned)__cvta_generic_to_shared(&mbar[parity])),
-                   "r"((unsigned)(48 * TRACK_CLUSTER * NW)) : "memory");
     // Each lane reads 4 adjacent pixels (one 8 B load of 4 colour bins) of 4 rows per step.  Rows are assigned by
     // ABSOLUTE frame row (a CTA keeps hitting its own L1 lines when the window shifts between passes).  The steps of
     // a pass (row group x 128-pixel column block) are software-pipelined: the four loads of step t+1 are issued
@@ -490,87 +448,6 @@ k_track(const uint16_t *__restrict__ bins, int W, int H, const int32_t *__restri
     const int xbeg = wx & ~3, xend = wx + ww;
     const int mine = crank * NW + warp;                          // rows with (wy+yy) % ROW_STRIDE == mine
     const int yy0 = (mine - (wy % ROW_STRIDE) + ROW_STRIDE) % ROW_STRIDE;
-#if HT_TRACK_LOOP2
-    if (vec4) {
-      // Round 2, call 16: under load a pass is bound by the instructions its warps issue (6 warps per scheduler), and a
-      // 16-pixel step cost ~330 of them - 50 for the four loads' address / predicate arithmetic, 16 selects for the window
-      // edge, the x factors (4 I2F.F64 + 4 DMUL) recomputed in every step.  Here: column blocks are the OUTER loop (x
-      // factors once per block, kept across its row groups), 32-bit row offsets, selects only in blocks that contain a
-      // window edge (warp-uniform), the row coordinate advanced by additions.
-      const int n_x = (xend - xbeg + 127) >> 7;
-      const int n_rg = (yy0 < wh) ? (wh - yy0 + 4 * ROW_STRIDE - 1) / (4 * ROW_STRIDE) : 0;
-      const int total = n_rg * n_x;
-      const uint16_t *col = px + (size_t)wy * W + xbeg + 4 * lane;
-      const uint32_t wsm_base = (uint32_t)__cvta_generic_to_shared(wsm);
-      const uint32_t rs = (uint32_t)ROW_STRIDE * (uint32_t)W;          // elements between two consecutive rows of this warp
-      auto issue = [&](int rg, int xi, uint2 (&v)[4]) {
-        const bool col_ok = xbeg + 4 * lane + 128 * xi < xend;
-        const int y0 = yy0 + 4 * rg * ROW_STRIDE;
-        const uint16_t *q = col + ((uint32_t)y0 * (uint32_t)W + 128u * (uint32_t)xi);
-#pragma unroll
-        for (int j = 0; j < 4; ++j)
-          v[j] = (col_ok && y0 + j * ROW_STRIDE < wh) ? __ldg(reinterpret_cast<const uint2 *>(q + (uint32_t)j * rs))
-                                                    : make_uint2(BIN_ZERO2, BIN_ZERO2);
-      };
-      double vx[4] = {0, 0, 0, 0}, vx2[4] = {0, 0, 0, 0};
-      unsigned in_mask = 0;
-      bool edge_any = true;
-      int cur_xi = -1;
-      auto consume = [&](int rg, int xi, const uint2 (&v)[4]) {
-        if (xi != cur_xi) {                                            // uniform over the warp
-          cur_xi = xi;
-          const int x4 = xbeg + 4 * lane + 128 * xi;
-          const double vx0 = (double)(x4 - wx);
-          in_mask = 0;
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            vx[i] = vx0 + (double)i;
-            vx2[i] = vx[i] * vx[i];
-            if (x4 + i >= wx && x4 + i < xend) in_mask |= 1u << i;
-          }
-          edge_any = __any_sync(0xffffffffu, in_mask != 15u);          // some lane of this block has pixels outside the window
-        }
-        const double vy0 = (double)(yy0 + 4 * rg * ROW_STRIDE);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          // a 128-pixel row segment whose entries are all ZERO (k_bins_mask: colours absent from the model; rows below
-          // the window) adds +0.0 to every sum: skip it with one vote (uniform over the warp)
-          if (!__any_sync(0xffffffffu, v[j].x != BIN_ZERO2 || v[j].y != BIN_ZERO2)) continue;
-          uint32_t b[4] = {v[j].x & 0xffffu, v[j].x >> 16, v[j].y & 0xffffu, v[j].y >> 16};   // table offsets (8 * bin)
-          if (edge_any) {   // pixels outside the window read the extra table entry wsm[4096] == +0.0
-#pragma unroll
-            for (int i = 0; i < 4; ++i) b[i] = ((in_mask >> i) & 1u) ? b[i] : BIN_ZERO;
-          }
-          double r0 = 0.0, r1 = 0.0, r2 = 0.0;
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            const double val = lds_f64(wsm_base + b[i]);
-            r0 += val;
-            r1 = fma(vx[i], val, r1);     // fused: this fast path is validated by trunc_ambiguous, the strict
-            r2 = fma(vx2[i], val, r2);    // reference order (separate multiply and add) is moments_serial
-          }
-          const double vy = vy0 + (double)(j * ROW_STRIDE);
-          a00 += r0; a10 += r1; a20 += r2;
-          a01 = fma(vy, r0, a01); a11 = fma(vy, r1, a11); a02 = fma(vy * vy, r0, a02);
-        }
-      };
-      // software pipeline over the steps (row group fastest inside a column block): the loads of step t+1 are in flight
-      // during the arithmetic of step t
-      uint2 va[4], vb[4];
-      int rg = 0, xi = 0;
-      if (total > 0) issue(0, 0, va);
-      for (int t = 0; t < total; t += 2) {
-        int rg1 = rg + 1, xi1 = xi;
-        if (rg1 == n_rg) { rg1 = 0; ++xi1; }
-        if (t + 1 < total) issue(rg1, xi1, vb);
-        consume(rg, xi, va);
-        int rg2 = rg1 + 1, xi2 = xi1;
-        if (rg2 == n_rg) { rg2 = 0; ++xi2; }
-        if (t + 2 < total) issue(rg2, xi2, va);
-        if (t + 1 < total) consume(rg1, xi1, vb);
-        rg = rg2; xi = xi2;
-      }
-#else
     if (vec4) {
       const int n_x = (xend - xbeg + 127) >> 7;
       const int n_rg = (yy0 < wh) ? (wh - yy0 + 4 * ROW_STRIDE - 1) / (4 * ROW_STRIDE) : 0;
@@ -634,7 +511,6 @@ k_track(const uint16_t *__restrict__ bins, int W, int H, const int32_t *__restri
         if (t + 1 < total) consume(rg1, xi1, vb);
         rg = rg2; xi = xi2;
       }
-#endif
     } else {
       for (int yy = yy0; yy < wh; yy += 4 * ROW_STRIDE) {
         double r[4][3];
@@ -654,43 +530,6 @@ k_track(const uint16_t *__restrict__ bins, int W, int H, const int32_t *__restri
       }
     }
     HT_PT_MARK(0);                     // pixel loop of this thread (loads, lookups, FMAs)
-    Mom msum = {0, 0, 0, 0, 0, 0};   // (MBAR) the window's moments, valid in thread 0
-    if (MBAR) {
-      a00 = warp_sum_all(a00); a10 = warp_sum_all(a10); a01 = warp_sum_all(a01);
-      a11 = warp_sum_all(a11); a20 = warp_sum_all(a20); a02 = warp_sum_all(a02);
-      const unsigned l_slot = (unsigned)__cvta_generic_to_shared(&wpart[MBAR ? parity : 0][MBAR ? crank * NW + warp : 0][0]);
-      const unsigned l_bar = (unsigned)__cvta_generic_to_shared(&mbar[parity]);
-      for (int idx = lane; idx < 6 * TRACK_CLUSTER; idx += 32) {   // lane -> (quantity q, destination CTA r)
-        const int q = idx % 6, r = idx / 6;
-        const double val = q == 0 ? a00 : q == 1 ? a10 : q == 2 ? a01 : q == 3 ? a11 : q == 4 ? a20 : a02;
-        unsigned r_slot, r_bar;
-        asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r_slot) : "r"(l_slot + 8u * (unsigned)q), "r"(r));
-        asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r_bar) : "r"(l_bar), "r"(r));
-        asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.b64 [%0], %1, [%2];"
-                     ::"r"(r_slot), "l"(__double_as_longlong(val)), "r"(r_bar) : "memory");
-      }
-      if (warp == 0) {
-        // wait for this pass's phase of the mbarrier (it is used every second pass: phase bit = bit 1 of pass_no)
-        const unsigned phase = (pass_no >> 1) & 1u;
-        unsigned done = 0;
-        for (int spin = 0; !done && spin < (1 << 26); ++spin)   // bounded: a protocol error must not hang the device
-          asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                       : "=r"(done) : "r"(l_bar), "r"(phase) : "memory");
-        if (!done) __trap();
-        // fixed-order sum of the C * NW slots: lane = (quantity q, residue g5 of the slot index mod 5), then the five
-        // partial sums of each quantity in ascending order - the same code on the same data in every CTA of the cluster
-        const int q = lane % 6, g5 = lane / 6;
-        double acc = 0.0;
-        if (g5 < 5)
-          for (int e = g5; e < TRACK_CLUSTER * NW; e += 5) acc += wpart[MBAR ? parity : 0][MBAR ? e : 0][q];
-        double t = acc;
-#pragma unroll
-        for (int j = 1; j < 5; ++j) t += __shfl_sync(0xffffffffu, acc, (q + 6 * j) & 31);
-        msum.m00 = __shfl_sync(0xffffffffu, t, 0); msum.m10 = __shfl_sync(0xffffffffu, t, 1);
-        msum.m01 = __shfl_sync(0xffffffffu, t, 2); msum.m11 = __shfl_sync(0xffffffffu, t, 3);
-        msum.m20 = __shfl_sync(0xffffffffu, t, 4); msum.m02 = __shfl_sync(0xffffffffu, t, 5);
-      }
-    } else {
     a00 = warp_sum(a00); a10 = warp_sum(a10); a01 = warp_sum(a01);
     a11 = warp_sum(a11); a20 = warp_sum(a20); a02 = warp_sum(a02);
     if (lane == 0) {
@@ -703,18 +542,16 @@ k_track(const uint16_t *__restrict__ bins, int W, int H, const int32_t *__restri
       const int q = tid % 6, r = tid / 6;
       double t = 0;
       for (int w8 = 0; w8 < NW; ++w8) t += red[w8][q];
-      cluster.map_shared_rank(&cpart[0][0][0], r)[(parity * TRACK_CLUSTER_MAX + crank) * 6 + q] = t;
+      cluster.map_shared_rank(&cpart[0][0][0], r)[(parity * TRACK_CLUSTER + crank) * 6 + q] = t;
     }
     if (TRACK_CLUSTER > 1) cluster.sync(); else __syncthreads();
-    }
     HT_PT_MARK(2);                     // cross-warp sum, remote stores, cluster barrier (wait for the slowest CTA)
     if (stepper) {
-      Mom m = msum;
-      if (!MBAR)
-        for (int r = 0; r < TRACK_CLUSTER; ++r) {
-          m.m00 += cpart[parity][r][0]; m.m10 += cpart[parity][r][1]; m.m01 += cpart[parity][r][2];
-          m.m11 += cpart[parity][r][3]; m.m20 += cpart[parity][r][4]; m.m02 += cpart[parity][r][5];
-        }
+      Mom m = {0, 0, 0, 0, 0, 0};
+      for (int r = 0; r < TRACK_CLUSTER; ++r) {
+        m.m00 += cpart[parity][r][0]; m.m10 += cpart[parity][r][1]; m.m01 += cpart[parity][r][2];
+        m.m11 += cpart[parity][r][3]; m.m20 += cpart[parity][r][4]; m.m02 += cpart[parity][r][5];
+      }
       bool exact = false;          // m is in the reference's strict summation order (moments_serial)
       bool fresh = true;           // m was computed by this pass (false: taken from the memo)
       int cw0 = win[0], cw1 = win[1], cw2 = win[2], cw3 = win[3];   // the window m belongs to
@@ -812,7 +649,6 @@ k_track(const uint16_t *__restrict__ bins, int W, int H, const int32_t *__restri
     }
     HT_PT_MARK(3);                     // scalar mean-shift step
     parity ^= 1;
-    ++pass_no;
     __syncthreads();
     HT_PT_MARK(4);                     // CTA barrier that publishes the next window
   }
@@ -823,7 +659,7 @@ k_track(const uint16_t *__restrict__ bins, int W, int H, const int32_t *__restri
     }
     if (stats) {
       atomicAdd(&stats[0], st_pass); atomicAdd(&stats[1], st_serial);
-      atomicAdd(&stats[2], st_px); atomicAdd(&stats[3], (unsigned long long)(call - call0));
+      atomicAdd(&stats[2], st_px); atomicAdd(&stats[3], (unsigned long long)call);
       atomicAdd(&stats[4], st_memo_sh);
     }
     state[slot] = s;
@@ -836,17 +672,12 @@ k_track(const uint16_t *__restrict__ bins, int W, int H, const int32_t *__restri
       for (int i = 0; i < 5; ++i) trace[trace_stride + 8 * (size_t)k + i] = (unsigned long long)pt_acc[i];
 #endif
     }
-    if (bailed) {   // phase B continues this stream from call `call`
-      calls_done[k] = call;
-      bail_list[atomicAdd(bail_count, 1)] = k;
-    } else {
-      int32_t *o = out_objs + 6 * (size_t)k;
-      o[0] = s.tx; o[1] = s.ty; o[2] = s.tw; o[3] = s.th;
-      *reinterpret_cast<double *>(o + 4) = s.angle;
-      if (out_windows) {
-        int32_t *w4 = out_windows + 4 * (size_t)k;
-        w4[0] = s.sx; w4[1] = s.sy; w4[2] = s.sw; w4[3] = s.sh;
-      }
+    int32_t *o = out_objs + 6 * (size_t)k;
+    o[0] = s.tx; o[1] = s.ty; o[2] = s.tw; o[3] = s.th;
+    *reinterpret_cast<double *>(o + 4) = s.angle;
+    if (out_windows) {
+      int32_t *w4 = out_windows + 4 * (size_t)k;
+      w4[0] = s.sx; w4[1] = s.sy; w4[2] = s.sw; w4[3] = s.sh;
     }
   }
   if (TRACK_CLUSTER > 1) cluster.sync();  // no CTA may exit while another one can still address its shared memory

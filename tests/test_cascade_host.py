@@ -87,8 +87,6 @@ def test_partial_quad_and_forced_ties(st, blob):
         assert base[f] == want_raw(frames[f], blob) and base[f]
     # every integer / truth-table decision replaced by the reference's ordered fp64 adds: same lists
     assert run(st, blob, frames, W, H, force_ties=3) == base
-    # stage 2 in quad form (the HT_QUAD_STAGES=3 build): same lists
-    assert run(st, blob, frames, W, H, quad_stages=3) == base
 
 
 def test_bench_resolution_frame(st, blob):

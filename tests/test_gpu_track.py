@@ -182,7 +182,7 @@ def test_track_odd_width_scalar_path(ctx, blob):
     assert abs(objs[0]["angle"] - want["angle"]) <= 1e-4 and wins[0] == ot.search_window()
 
 
-@pytest.mark.parametrize("env", [{}, {"HT_TRACK_HEAVY": "8"}, {"HT_TRACK_NT": "128", "HT_TRACK_HEAVY": "4,4"},
+@pytest.mark.parametrize("env", [{}, {"HT_TRACK_HEAVY": "8"}, {"HT_TRACK_HEAVY": "4,4"},
                                  {"HT_TRACK_LPT": "0"}, {"HT_TRACK_MEMO": "0"}])
 def test_scheduled_launch_orders_do_not_change_results(blob, env, monkeypatch):
     """>= 128 streams: k_track runs the streams longest-window-first (optionally the largest ones on a bigger cluster

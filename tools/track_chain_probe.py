@@ -44,7 +44,7 @@ def main():
         f = synth.frame(fid, W, H)
         for n in (1, 16):
             batch = np.stack([f] * n)
-            for c in (1, 2, 4, 8):
+            for c in (2, 4, 8):
                 os.environ["HT_TRACK_CLUSTER"] = str(c)
                 ms, st = run(batch)
                 print(f"frame {fid} n={n} cluster={c}: track {ms:.3f} ms  stats={st}", flush=True)
